@@ -1,6 +1,6 @@
 """Benchmark of the denoising hot path (BASELINE.json metric: denoise-steps/sec, 16 f x 512^2 SD-1.5 UNet3D).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR] [--profile-dir DIR]
 
 One "step" = one loop body of the reference pipeline (pipelines/pipeline_videoswap.py:556-587): CFG batch
 duplication, AnimateDiffUNet3DModel forward on [2,4,16,64,64], CFG combine, DDIM update.  Workload = BASELINE config
@@ -11,6 +11,13 @@ CFG halves (one all-gather of the noise predictions per step), N = 4 / 8 CFG x 2
 all-reduces + frames<->pixels all-to-all around the motion modules, NCCL over NVLink, captured in the CUDA graph);
 `value` = steps of that one video per second.  --mode replicas: one video per rank (weak scaling, no data-path
 collective).  Barrier + device timing, max over ranks.
+
+The benchmark writes nothing into the source tree (it may be read-only): --dump-outputs DIR writes the latents the timed
+path returned in its last step as DIR/latents.npy (float32; one file per rank, latents_rank<r>.npy, when N > 1), and
+--profile-dir DIR the per-shape kernel profile CSV.  Weights and inputs come from fixed seeds, so two builds run with the
+same arguments can be compared output for output.  The GroupNorm statistics are summed with float atomics, so two runs of
+one build already differ in the last bits: 76 dB PSNR between the dumps of two `--steps 10 --warmup 3` runs (B200, 1000 W
+power limit).
 """
 from __future__ import annotations
 
@@ -33,6 +40,21 @@ UNIT = "steps/s"
 FLOP_PER_STEP = 35.26e12          # algorithmic FLOPs of one CFG step at this config (SURVEY.md 8d)
 FRAMES, LATENT = 16, 64
 CATS = ["gemm", "conv3x3", "attention", "temporal_attention", "groupnorm", "layernorm", "other"]
+DUMP_LIMIT = 64 << 20             # bytes of --dump-outputs per run
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Writes each tensor as <out_dir>/<name>.npy in float32.  When they exceed `limit` bytes in all, each is replaced by
+    the same fixed, seeded sample of its flattened elements (sorted positions), so that runs stay comparable."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            keep = a.size * limit // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def peaks():
@@ -207,7 +229,13 @@ def main():
                          "default) or independent videos per rank (weak scaling)")
     ap.add_argument("--option", action="append", default=[], help="kernel A/B switch name=value (vs_set_option)")
     ap.add_argument("--tag", default="", help="suffix of the per-shape profile CSV")
+    ap.add_argument("--profile-dir", help="write the per-shape profile CSV (profile_shapes_n<N><tag>.csv) of the eager pass here")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the latents of the last timed step as DIR/latents.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl native (the reference arm times a CPU sample, not the step)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -295,12 +323,13 @@ def main():
         a, b, c = C.c_double(), C.c_double(), C.c_longlong()
         _lib.call("vs_profile_collect", ci, C.byref(a), C.byref(b), C.byref(c))
         prof[name] = {"ms_per_step": a.value / K, "work_per_step": b.value / K, "launches_per_step": c.value / K}
-    if rank == 0:
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        lib.vs_profile_dump(os.path.join(ROOT, "gpurun_out", f"profile_shapes_n{world}{args.tag}.csv").encode())
+    if rank == 0 and args.profile_dir:
+        os.makedirs(args.profile_dir, exist_ok=True)
+        _lib.call("vs_profile_dump", os.path.join(args.profile_dir, f"profile_shapes_n{world}{args.tag}.csv").encode())
     lib.vs_profile_reset()
     finite = bool(torch.isfinite(lat).all().item())
     ms_eager = ms
+    last_out = lat.clone() if args.dump_outputs else None    # the timed path's result when there is no graph
 
     # ---------------- timed region 1b (the reported `value`): the same step captured in a CUDA graph and replayed
     gstep = None
@@ -319,6 +348,8 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)
+        if args.dump_outputs:
+            last_out = lat.clone()           # the graph's output buffer is overwritten by the end-to-end pass below
         if world > 1:
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -465,9 +496,12 @@ def main():
         else:
             out["cpu_baseline"] = None
         print(json.dumps(out))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latents" if world == 1 else f"latents_rank{rank}": last_out}, DUMP_LIMIT // world)
     if world > 1:
         dist.destroy_process_group()
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True    # the package is imported inside main(): no __pycache__ in the tree the benchmark runs from
     main()

@@ -8,6 +8,9 @@ REFERENCE's own functions read from /root/reference:
 
 The UNet state dict is the seeded tiny configuration of the CPU tests (re-created from its seed by the test, not stored); the
 fixture stores the LoRA, and for the merged result the touched tensors of a few named keys plus a digest over all of them.
+A second fixture, tests/golden/edlora_merge_pair.pt, holds merge_lora_into_weight's result for two full-size weights (a
+Linear and a 1x1 conv, inputs re-created from their seed by the test): every MERGE_STRIDE-th element of each merged tensor
+and its float64 sum and sum of squares (the whole tensors would exceed 1 MB).
     python -m oracle.make_golden_formats"""
 import ast
 import hashlib
@@ -20,10 +23,12 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 OUT = os.path.join(ROOT, "tests", "golden", "formats.pt")
+MERGE_OUT = os.path.join(ROOT, "tests", "golden", "edlora_merge_pair.pt")
 REF = os.environ.get("VIDEOSWAP_REFERENCE", "/root/reference")
 
 TINY = dict(boc=(32, 64, 128, 128), ctx=64, groups=8)
 RANK, ALPHA = 4, 0.6
+MERGE_STRIDE = 61
 
 
 def function_from_file(path, name, env=None):
@@ -74,10 +79,43 @@ def digest(sd, keys):
     return h.hexdigest()
 
 
-def main():
+def merge_pair_inputs(seed=7):
+    """Two weights of the full UNet, a Linear and a 1x1 conv, with rank-4 LoRA pairs (base, lora)."""
+    k1 = "down_blocks.0.attentions.0.transformer_blocks.0.attn2.to_k.weight"
+    k2 = "down_blocks.0.attentions.0.proj_in.weight"                       # 4-D 1x1 conv weight
+    g = torch.Generator().manual_seed(seed)
+    base = {k1: torch.randn((320, 768), generator=g), k2: torch.randn((320, 320, 1, 1), generator=g)}
+    lora = {k1.replace("to_k.weight", "to_k.lora_down.weight"): torch.randn((RANK, 768), generator=g),
+            k1.replace("to_k.weight", "to_k.lora_up.weight"): torch.randn((320, RANK), generator=g),
+            k2.replace("proj_in.weight", "proj_in.lora_down.weight"): torch.randn((RANK, 320, 1, 1), generator=g),
+            k2.replace("proj_in.weight", "proj_in.lora_up.weight"): torch.randn((320, RANK, 1, 1), generator=g)}
+    return base, lora
+
+
+def merge_pair_summary(merged):
+    """What edlora_merge_pair.pt keeps of a merged tensor."""
+    flat = merged.reshape(-1)
+    return {"shape": tuple(merged.shape), "sample": flat[::MERGE_STRIDE].clone(),
+            "sum": float(flat.double().sum()), "sumsq": float((flat.double() ** 2).sum())}
+
+
+def reference_convert():
     spec = importlib.util.spec_from_file_location("ref_convert_edlora", os.path.join(REF, "videoswap/utils/convert_edlora_to_diffusers.py"))
     ref = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref)
+    return ref
+
+
+def write_merge_pair(ref):
+    base, lora = merge_pair_inputs()
+    merged = ref.merge_lora_into_weight(base, lora, model_type="unet", alpha=ALPHA)
+    torch.save({"alpha": ALPHA, "stride": MERGE_STRIDE, "merged": {k: merge_pair_summary(merged[k]) for k in base}}, MERGE_OUT)
+    print("wrote", MERGE_OUT, os.path.getsize(MERGE_OUT), "bytes")
+
+
+def main():
+    ref = reference_convert()
+    write_merge_pair(ref)
     select_frame_idx = function_from_file(os.path.join(REF, "videoswap/data/frame_point_dataset.py"), "select_frame_idx")
     bind_concept_prompt = function_from_file(os.path.join(REF, "videoswap/utils/edlora_util.py"), "bind_concept_prompt")
 

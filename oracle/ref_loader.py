@@ -1,7 +1,7 @@
-"""TEST INFRASTRUCTURE ONLY.  Imports the reference's OWN model files, unmodified, from /root/reference
-through oracle/diffusers_stub (the reference's `diffusers==0.19.3` dependency is not installable offline).
-Only usable in the authoring container (/root/reference does not exist on the GPU box); used by
-oracle/make_golden.py to pin oracle/unet3d_oracle.py and by tests that skip when the reference is absent."""
+"""TEST INFRASTRUCTURE ONLY.  Imports the reference's OWN model files, unmodified, from a checkout of the reference
+project (REFERENCE_ROOT, env VIDEOSWAP_REFERENCE) through oracle/diffusers_stub (the reference's `diffusers==0.19.3`
+dependency is not installable offline).  Used by the oracle/make_golden*.py scripts that write the fixtures under
+tests/golden/; no test needs the reference itself."""
 import importlib
 import os
 import sys

@@ -89,6 +89,22 @@ def test_product_never_imports_oracle():
                 assert "/root/reference" not in text, f
 
 
+def test_bench_dump_outputs_float32_and_seeded_sample(tmp_path):
+    """bench.py --dump-outputs: float32 .npy files; over the byte limit, the same sorted sample positions every run."""
+    import numpy as np
+    import bench
+    x = torch.arange(4 * 16, dtype=torch.float16).reshape(4, 16)
+    bench.dump_outputs(str(tmp_path / "full"), {"latents": x})
+    a = np.load(tmp_path / "full" / "latents.npy")
+    assert a.dtype == np.float32 and a.shape == (4, 16) and np.array_equal(a, x.float().numpy())
+    for run in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / run), {"latents": x, "eps": 2 * x}, limit=128)
+    s1, s2 = np.load(tmp_path / "s1" / "latents.npy"), np.load(tmp_path / "s2" / "latents.npy")
+    assert s1.dtype == np.float32 and s1.size == 16 and np.array_equal(s1, s2)
+    assert np.all(np.diff(s1) > 0) and set(s1.tolist()) <= set(range(64))       # sorted positions of arange = values
+    assert np.array_equal(np.load(tmp_path / "s1" / "eps.npy"), 2 * s1)           # every array sampled at the same positions
+
+
 def test_registry_names():
     assert V.build_model("AnimateDiffUNet3DModel") is V.AnimateDiffUNet3DModel
     assert V.build_model("UNet3DConditionModel") is V.AnimateDiffUNet3DModel
@@ -221,7 +237,8 @@ def test_on_disk_formats_of_the_callers_load_unchanged(tmp_path):
     ('.pos_encoder' -> '.processor.pos_encoder') match our keys exactly; (ii) adapter.pth is the SparsePointAdapter
     state_dict; (iii) TAP.pth is the dict frame_point_dataset.py:66-70 turns into `conditions`; (iv) an ED-LoRA '.pth'
     ({'params': {'unet': {...lora_down / lora_up...}}}) merges through state_dict()/load_state_dict() exactly like
-    convert_edlora_to_diffusers.py:70-76 (run with the reference's own function when /root/reference is present)."""
+    convert_edlora_to_diffusers.py:70-76 (tests/golden/edlora_merge_pair.pt: the reference's own function on the same seeded
+    inputs, oracle/make_golden_formats.py)."""
     m = V.AnimateDiffUNet3DModel(init="empty")
     keys = set(m.state_dict().keys())
     motion = {k for k in keys if ".motion_modules." in k}
@@ -243,23 +260,20 @@ def test_on_disk_formats_of_the_callers_load_unchanged(tmp_path):
     cond = {"pred_tracks": t["pred_tracks"], "point_embedding": t["point_embedding"], "point_name2id": t["point_name2id"],
             "img_size": (512, 512), "index_list": [t["point_name2id"]["nose"]]}
     assert cond["pred_tracks"].shape == (16, 5, 2) and cond["point_embedding"].shape[1] == 1280
-    # ED-LoRA merge on two layers (rank 4), restated and -- when available -- through the reference's own function
+    # ED-LoRA merge on two layers (rank 4), restated and compared with the reference's own function's result
+    from oracle.make_golden_formats import merge_pair_inputs, merge_pair_summary
     k1 = "down_blocks.0.attentions.0.transformer_blocks.0.attn2.to_k.weight"
     k2 = "down_blocks.0.attentions.0.proj_in.weight"                       # 4-D 1x1 conv weight
-    base = {k1: torch.randn(320, 768), k2: torch.randn(320, 320, 1, 1)}
-    lora = {k1.replace("to_k.weight", "to_k.lora_down.weight"): torch.randn(4, 768), k1.replace("to_k.weight", "to_k.lora_up.weight"): torch.randn(320, 4),
-            k2.replace("proj_in.weight", "proj_in.lora_down.weight"): torch.randn(4, 320, 1, 1),
-            k2.replace("proj_in.weight", "proj_in.lora_up.weight"): torch.randn(320, 4, 1, 1)}
+    base, lora = merge_pair_inputs()
     want = {k1: base[k1] + 0.6 * lora[k1.replace("to_k.weight", "to_k.lora_up.weight")] @ lora[k1.replace("to_k.weight", "to_k.lora_down.weight")],
             k2: base[k2] + 0.6 * (lora[k2.replace("proj_in.weight", "proj_in.lora_up.weight")].squeeze() @
                                   lora[k2.replace("proj_in.weight", "proj_in.lora_down.weight")].squeeze())[..., None, None]}
-    from oracle.ref_loader import reference_available
-    if reference_available():
-        import importlib
-        from oracle.ref_loader import load_reference
-        load_reference()
-        conv = importlib.import_module("videoswap.utils.convert_edlora_to_diffusers")
-        got = conv.merge_lora_into_weight(base, lora, model_type="unet", alpha=0.6)
-        assert all(torch.allclose(got[k], want[k], atol=1e-5) for k in want)
+    gold = torch.load(os.path.join(ROOT, "tests", "golden", "edlora_merge_pair.pt"))
+    assert gold["alpha"] == 0.6 and sorted(gold["merged"]) == sorted(want)
+    for k in want:
+        got, ref = merge_pair_summary(want[k]), gold["merged"][k]
+        assert got["shape"] == ref["shape"] and torch.allclose(got["sample"], ref["sample"], atol=1e-5), k
+        assert abs(got["sum"] - ref["sum"]) <= 1e-5 * want[k].numel(), k
+        assert abs(got["sumsq"] - ref["sumsq"]) <= 1e-6 * ref["sumsq"], k
     m.load_state_dict(want, strict=False)                                   # the merged dict goes back through load_state_dict
     assert torch.allclose(m.state_dict()[k1], want[k1]) and m._dirty       # ... and marks the packed weights stale
